@@ -182,6 +182,16 @@ def _emit(saved_fd, line: dict):
     os.write(saved_fd, (json.dumps(line) + "\n").encode())
 
 
+def dump_outputs(path, results):
+    """What each timed path returned to its caller in its last timed step — the suggestion: global candidate index, acquisition
+    value, posterior mean and std — as DIR/<path>_<field>.npy, one float64 array of one element per field (the index is exact in
+    float64).  The inputs are seeded, so two builds run with the same arguments can be compared file by file."""
+    os.makedirs(path, exist_ok=True)
+    for name, best in results.items():
+        for field in ("index", "value", "mu", "std"):
+            np.save(os.path.join(path, f"{name}_{field}.npy"), np.array([getattr(best, field)], dtype=np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -195,7 +205,12 @@ def main():
     ap.add_argument("--k-span", type=int, default=0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the suggestion of the last timed step of the device and e2e paths to DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed: it needs --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -280,6 +295,8 @@ def main():
     clocks = sampler.stop() if rank == 0 else None
     tims = tims[-args.steps:]
     assert best_h.index == best.index, "host and device paths disagree on the argmax"
+    if args.dump_outputs and rank == 0:   # after the exchange every rank holds the same global suggestion
+        dump_outputs(args.dump_outputs, {"device": best, "e2e": best_h})
     chunks = tims[-1]["chunks"]
     launches = sum(t["launches"] for t in tims)
     mean = lambda k: float(np.mean([t[k] for t in tims]))   # noqa: E731
